@@ -10,10 +10,11 @@ memory; strong scaling, `parity_vs_n1` = max |sharded - single-GPU| of the step'
 The line also carries the second half of BASELINE's metric: `vae_decode` (768p causal-VAE decode, frames/s + conv roofline)
 and `video_e2e` (the whole 768p / 10 s pyramidal sampler + decode, frames/s), and two baselines timed in the same run: the
 reference algorithm on the host cores (`cpu_baseline`) and the UNMODIFIED reference modules in eager PyTorch bf16 on the
-same B200 (`gpu_eager_baseline`, from the copy staged in baseline/_ref).
+same B200 (`gpu_eager_baseline`, when oracle/pin/stage_reference.py has staged the reference in oracle/_ref).
 
   python bench.py [--gpus N] [--steps K] [--warmup W]           our arm (CUDA kernels through the C-ABI)
   python bench.py --impl reference ...                           the reference algorithm's CPU path (oracle port), host cores
+  python bench.py ... --dump-outputs DIR                         also write the last timed step's output to DIR/<name>.npy
 
 Prints ONE JSON line (rank 0).  See DESIGN.md §Measurement for the definitions of value / e2e / roofline / cpu_baseline.
 """
@@ -105,6 +106,17 @@ def measured_peaks():
     return {"tflops_sustained": 1400.0, "tflops_burst": 1590.0, "hbm_gbs": 6650.0, "source": "fallback (B200_PROFILING.md)"}
 
 
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: the arrays the timed path returned in its last timed step, as DIR/<name>.npy in float32 (a few MB),
+    so that two builds can be compared output for output: inputs and weights come from fixed seeds, identical from run to
+    run with the same arguments."""
+    import numpy as np
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(d / f"{name}.npy", t.detach().float().cpu().numpy())
+
+
 # ----------------------------------------------------------------------------------------------------------------------
 def cpu_reference_sample(n_double=1, n_single=2, threads=None, repeats=1):
     """Time the reference algorithm's CPU path (oracle port, fp32) on a bounded sample; returns tokens/s extrapolated to
@@ -128,11 +140,11 @@ def cpu_reference_sample(n_double=1, n_single=2, threads=None, repeats=1):
     with torch.no_grad():
         for _ in range(repeats):
             t0 = time.perf_counter()
-            FO.flux_forward(params, cfg, clips, t, enc, mask, pooled)
+            out = FO.flux_forward(params, cfg, clips, t, enc, mask, pooled)
             times.append(time.perf_counter() - t0)
     dt = sorted(times)[len(times) // 2]
     full = dt * (8 + 16) / (n_double + n_single)   # block cost dominates; embedders/head are <1 %
-    return {"tokens_per_s": b * s / full, "sample_s": dt, "threads": threads, "tokens": b * s,
+    return {"tokens_per_s": b * s / full, "sample_s": dt, "threads": threads, "tokens": b * s, "out": out,
             "sample": (f"oracle port (PyTorch fp32, {threads} threads): {n_double} double + {n_single} single miniFLUX blocks at "
                        f"B={b}, S={s} (768p unit 30 / stage 0 sequence), time x{(8 + 16) / (n_double + n_single):.0f} to the "
                        f"24-block forward")}
@@ -148,8 +160,10 @@ def run_reference(args):
     for _ in range(max(1, args.warmup)):
         cpu_reference_sample(repeats=1)             # untimed: page-in, thread pool
     t0 = time.perf_counter()
-    vals = [cpu_reference_sample(repeats=1) for _ in range(max(1, args.steps))]
+    vals = [cpu_reference_sample(repeats=1) for _ in range(args.steps)]
     wall = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"reference_sample_out": vals[-1]["out"]})
     tok = vals[0]["tokens"]
     mean_full_s = sum(v["tokens"] / v["tokens_per_s"] for v in vals) / len(vals)     # extrapolated 24-block seconds per step
     value = tok / mean_full_s
@@ -169,14 +183,14 @@ def run_reference(args):
 
 
 def gpu_eager_reference(dev, host, steps=2):
-    """The UNMODIFIED reference `PyramidFluxTransformer` (baseline/_ref copy through oracle/pin/ref_shim.py) in eager PyTorch
+    """The UNMODIFIED reference `PyramidFluxTransformer` (oracle/_ref copy through oracle/pin/ref_shim.py) in eager PyTorch
     under bf16 autocast on this GPU: the full 8+16-block forward at the bench shape, dense [B,1,S,S] bool mask + SDPA as the
     reference builds them (F:318-350, B:363-365).  A reported baseline (SURVEY.md §8d), never on the product path."""
     import torch
     try:
         from oracle.pin import ref_shim
         if not ref_shim.reference_available():
-            return {"unavailable": "reference packages not staged in baseline/_ref (oracle/pin/stage_reference.py)"}
+            return {"unavailable": "reference packages not staged in oracle/_ref (oracle/pin/stage_reference.py)"}
         ref_shim.install()
         from pyramid_dit.flux_modules import PyramidFluxTransformer
         with torch.device(dev):
@@ -369,10 +383,10 @@ def run_mmdit(args):
         n0 = _lib.launch_count()
         s_.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         e_.record()
         torch.cuda.synchronize()
-        return s_.elapsed_time(e_) / steps, _lib.launch_count() - n0
+        return s_.elapsed_time(e_) / steps, _lib.launch_count() - n0, out
 
     for _ in range(max(args.warmup, 3)):
         step_resident()
@@ -380,11 +394,13 @@ def run_mmdit(args):
     sampler.start()
     time.sleep(0.25)
     t0 = time.time()
-    ms, launches = timed(step_resident, args.steps)
+    ms, launches, step_out = timed(step_resident, args.steps)
     t1 = time.time()
     clocks = sampler.stop(t0, t1)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"mmdit_step_out": step_out})
     step_e2e()
-    ms_e2e, _ = timed(step_e2e, args.steps)
+    ms_e2e, _, _ = timed(step_e2e, args.steps)
     plan = model.last_plan
     d = cfg.inner_dim
     tokens = b * plan.seq
@@ -609,7 +625,7 @@ def run_ours(args):
         s.record()
         h0 = time.perf_counter()
         for _ in range(steps):
-            fn()
+            out = fn()
         host_ms["last"] = (time.perf_counter() - h0) * 1e3 / steps     # host time to ENQUEUE a step (no sync inside)
         e.record()
         barrier()
@@ -619,7 +635,7 @@ def run_ours(args):
             tt = torch.tensor([ms], device=dev)
             dist.all_reduce(tt, op=dist.ReduceOp.MAX)
             ms = float(tt.item())
-        return ms / steps, launches
+        return ms / steps, launches, out
 
     for _ in range(max(args.warmup, 3)):
         step_resident()
@@ -630,14 +646,17 @@ def run_ours(args):
     sampler.start()
     time.sleep(0.25)
     t0 = time.time()
-    ms_step, launches = timed(step_resident, args.steps, events=False)
+    ms_step, launches, step_out = timed(step_resident, args.steps, events=False)
     host_enqueue_ms = host_ms["last"]
     t1 = time.time()
     clocks = sampler.stop(t0, t1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"dit_step_out": step_out})
+    del step_out
     # the timed region above carries no per-launch instrumentation (graph replay, or plain host launches with --no-graph);
     # the dominant kernel's launch durations come from the same number of host-launched steps run right after it, with CUDA
     # events around each attention launch
-    ms_eager, _ = timed(step_resident, args.steps, events=True)
+    ms_eager, _, _ = timed(step_resident, args.steps, events=True)
     # dominant kernel: the masked attention; per-launch duration from CUDA events recorded around each launch
     ev = model.attn_events or []
     model.attn_events = None
@@ -650,7 +669,7 @@ def run_ours(args):
     attn_avg = sum(attn_ms) / max(1, len(attn_ms))
     step_e2e()
     step_e2e()
-    ms_e2e, _ = timed(step_e2e, args.steps)
+    ms_e2e, _, _ = timed(step_e2e, args.steps)
     # per-kernel-family breakdown of ONE extra (untimed-for-the-metric) step, CUDA events around every launch
     model.timer.enabled = True
     model.attn_events = []
@@ -766,7 +785,11 @@ def main():
     ap.add_argument("--no-vae", action="store_true", help="skip the VAE decode leg")
     ap.add_argument("--no-video", action="store_true", help="skip the 768p/10s end-to-end sampler + decode leg (~1 min at N=1)")
     ap.add_argument("--no-eager", action="store_true", help="skip the reference-eager-on-GPU baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     elif args.model == "mmdit":

@@ -1,9 +1,13 @@
-"""Generate tests/golden/* by running the UNMODIFIED reference (imported from /root/reference through ref_shim).
+"""Generate tests/golden/* by running the UNMODIFIED reference (imported through ref_shim).
 
-Run in the build container only:  python oracle/pin/make_golden.py [flux] [block] [sched] [vae] [loop]
-The GPU box has no /root/reference; it only sees the small fixtures this script commits under tests/golden/.
+    PF_REFERENCE_ROOT=/path/to/Pyramid-Flow python oracle/pin/make_golden.py [flux] [block] [sched] [vae] [vae_encoder] [sampler] [sampler_i2v] [mmdit]
+    python oracle/pin/make_golden.py dropin         (needs a CUDA GPU; the reference staged by oracle/pin/stage_reference.py)
+
+The tests never import the reference; they only see the small fixtures this script writes under tests/golden/.
 Inputs and parameters are regenerated from seeds by the tests (torch CPU generators are deterministic), so the fixtures
-hold the reference OUTPUTS plus the exact inputs for safety.
+hold the reference OUTPUTS plus the exact inputs for safety.  Files stay under 1 MB: a large output is stored as the
+fixed strided sample `t.flatten()[::SAMPLE_STRIDE]` (the stride is coprime with every axis length, so each row, column and
+channel is sampled).
 """
 from __future__ import annotations
 
@@ -22,6 +26,7 @@ from oracle import flux_oracle as FO  # noqa: E402
 GOLD = ROOT / "tests" / "golden"
 GOLD.mkdir(parents=True, exist_ok=True)
 
+SAMPLE_STRIDE = 13
 SMALL_CFG = dict(num_layers=2, num_single_layers=2, num_attention_heads=4, attention_head_dim=64, in_channels=64,
                  joint_attention_dim=128, pooled_projection_dim=64)
 
@@ -145,7 +150,9 @@ def make_vae():
     print("vae:", full.shape, float(full.abs().mean()), "chunk1 diff", float((full - chunk1).abs().max()),
           "chunk2 diff", float((full - chunk2).abs().max()), "tiled diff", float((full - tiled).abs().max()))
     torch.save({"cfg": VAE_SMALL, "param_seed": 0, "z": z, "full": full, "chunk1_maxdiff": float((full - chunk1).abs().max()),
-                "chunk2_maxdiff": float((full - chunk2).abs().max()), "tiled32": tiled}, GOLD / "vae_small.pt")
+                "chunk2_maxdiff": float((full - chunk2).abs().max()), "tiled32_shape": tuple(tiled.shape),
+                "tiled32_stride": SAMPLE_STRIDE, "tiled32_sample": tiled.flatten()[::SAMPLE_STRIDE].clone()},
+               GOLD / "vae_small.pt")
 
 
 def make_vae_encoder():
@@ -303,6 +310,88 @@ def make_sampler_i2v():
     torch.save({"cfg": SMALL_CFG, "param_seed": 0, "enc": enc, "mask": mask, "pooled": pooled, "noises": noises,
                 "latent_seed": 5, "latents": lat, "image_tensor": FakeVae.seen[0], "image_latent_raw": image_latent_raw,
                 "args": dict(height=128, width=128, **args)}, GOLD / "sampler_i2v_small.pt")
+
+
+DROPIN_VAE_DEC = dict(block_out_channels=(64, 64, 128, 128), layers_per_block=(1, 1, 1, 1))
+DROPIN_VAE_ENC = dict(block_out_channels=(64, 64, 128, 128), layers_per_block=(1, 1, 1, 1))
+
+
+def make_dropin():
+    """The UNMODIFIED reference pipeline `PyramidDiTForVideoGeneration` with the reference's own modules on a CUDA GPU, bf16
+    weights under torch.autocast (the README's way of running it): generate() final latents on the inputs of
+    sampler_small.pt, and generate_i2v() -> decode_latent() uint8 frames on those of sampler_i2v_small.pt (tiny reference
+    DiT, small reference VAE with synthetic weights).  tests/test_dropin_gpu.py drives the B200 modules, built through
+    from_reference() from the module configs stored here, on the same inputs and compares with these outputs."""
+    import numpy as np
+    from PIL import Image
+    from diffusion_schedulers import PyramidFlowMatchEulerDiscreteScheduler
+    from oracle import vae_oracle as VO
+    from pyramid_dit import PyramidDiTForVideoGeneration
+    from pyramid_dit.flux_modules import PyramidFluxTransformer
+    from video_vae import CausalVideoVAE
+    dev = torch.device("cuda:0")
+
+    def ref_dit(g):
+        dit = PyramidFluxTransformer(**g["cfg"]).eval()
+        dit.load_state_dict(FO.synthetic_flux_params(FO.FluxConfig(**g["cfg"]), seed=g["param_seed"]), strict=True)
+        return dit.to(dev, torch.bfloat16)
+
+    def make_pipe(g, dit, vae):
+        class FakeText:   # generate() asks for the prompt first, then for the negative prompt (P:1066-1067)
+            calls = 0
+
+            def __call__(self, prompt, device):
+                i = 1 if self.calls % 2 == 0 else 0
+                self.calls += 1
+                return (g["enc"][i:i + 1].to(dev).bfloat16(), g["mask"][i:i + 1].to(dev),
+                        g["pooled"][i:i + 1].to(dev).bfloat16())
+
+        pipe = object.__new__(PyramidDiTForVideoGeneration)
+        pipe.dit, pipe.vae, pipe.text_encoder = dit, vae, FakeText()
+        pipe.scheduler = PyramidFlowMatchEulerDiscreteScheduler(shift=1.0, stages=3, stage_range=[0, 1 / 3, 2 / 3, 1], gamma=1 / 3)
+        pipe.stages = [1, 2, 4]
+        pipe.frame_per_unit = 1
+        pipe.model_name = "pyramid_flux"
+        pipe.sequential_offload_enabled = False
+        pipe.downsample = 8
+        pipe.vae_shift_factor, pipe.vae_scale_factor = -0.04, 1 / 1.8726
+        pipe.vae_video_shift_factor, pipe.vae_video_scale_factor = -0.2343, 1 / 3.0986
+        noises = [n.clone() for n in g["noises"]]
+        pipe.sample_block_noise = lambda bs, ch, temp, height, width: noises.pop(0)
+        return pipe
+
+    g = torch.load(GOLD / "sampler_small.pt", weights_only=False)
+    dit = ref_dit(g)
+    with torch.no_grad(), torch.autocast("cuda", dtype=torch.bfloat16):
+        lat = make_pipe(g, dit, None).generate(prompt="x", generator=torch.Generator().manual_seed(g["latent_seed"]),
+                                               output_type="latent", save_memory=True, **g["args"])
+
+    gi = torch.load(GOLD / "sampler_i2v_small.pt", weights_only=False)
+    dcfg, ecfg = VO.VaeDecoderConfig(**DROPIN_VAE_DEC), VO.VaeEncoderConfig(**DROPIN_VAE_ENC)
+    vae = CausalVideoVAE(encoder_out_channels=16, decoder_in_channels=16, encoder_block_out_channels=ecfg.block_out_channels,
+                         encoder_layers_per_block=ecfg.layers_per_block, decoder_block_out_channels=dcfg.block_out_channels,
+                         decoder_layers_per_block=dcfg.layers_per_block).eval()
+    sd = vae.state_dict()
+    new = {**VO.synthetic_vae_params(dcfg, seed=4), **VO.synthetic_vae_params(ecfg, seed=5)}
+    assert set(new) == set(sd), set(new) ^ set(sd)
+    # latent_dist.sample() draws from the global RNG (D:381-389): pin log-variance at -30 so the image latent is its mean
+    new["quant_conv.conv.weight"][16:] = 0
+    new["quant_conv.conv.bias"][16:] = -30.0
+    vae.load_state_dict(new, strict=True)
+    vae = vae.to(dev, torch.bfloat16)
+    vae.enable_tiling()
+    img = Image.fromarray((gi["image_tensor"][0, :, 0].permute(1, 2, 0) * 127.5 + 127.5).round().clamp(0, 255).byte().numpy())
+    args = {k: v for k, v in gi["args"].items() if k not in ("height", "width")}
+    torch.manual_seed(123)
+    with torch.no_grad(), torch.autocast("cuda", dtype=torch.bfloat16):
+        out = make_pipe(gi, ref_dit(gi), vae).generate_i2v(prompt="x", input_image=img, output_type="pil", save_memory=True,
+                                                           generator=torch.Generator().manual_seed(gi["latent_seed"]), **args)
+    frames = torch.from_numpy(np.stack([np.asarray(f) for f in out]))
+    print("dropin:", lat.shape, float(lat.float().abs().mean()), "frames", tuple(frames.shape), float(frames.float().std()))
+    torch.save({"dit_config": dict(dit.config), "vae_config": dict(vae.config), "latents": lat.cpu(),
+                "frames_shape": tuple(frames.shape), "frames_stride": SAMPLE_STRIDE,
+                "frames_sample": frames.flatten()[::SAMPLE_STRIDE].clone(),
+                "device": torch.cuda.get_device_name(dev), "torch": torch.__version__}, GOLD / "dropin_gpu.pt")
 
 
 MMDIT_SMALL = dict(num_layers=3, num_attention_heads=4, attention_head_dim=64, in_channels=16, patch_size=2,

@@ -1,7 +1,7 @@
-"""Dependency shim so the UNMODIFIED reference (/root/reference) imports in this container.
+"""Dependency shim so the UNMODIFIED reference (a jy0205/Pyramid-Flow checkout) imports without its pip dependencies.
 
-TEST INFRASTRUCTURE, used only by oracle/pin/*.py (run in the build container where /root/reference exists) to pin
-the oracle restatement and to generate tests/golden/*.  Nothing shipped or measured imports this.
+TEST INFRASTRUCTURE, used by oracle/pin/make_golden.py to pin the oracle restatement and to generate tests/golden/*, and by
+bench.py's optional `gpu_eager_baseline` leg.  No test and no product module imports this.
 
 The image lacks diffusers / accelerate / timm / tensorboardX / IPython (SURVEY.md §8c).  The pieces of those packages
 the reference touches at import time are stubbed; the four that carry arithmetic are restated from the diffusers 0.30
@@ -25,9 +25,9 @@ import torch.nn.functional as F
 
 import os as _os
 
-# /root/reference in the build container; on the GPU box the byte-for-byte copy staged by oracle/pin/stage_reference.py
-_STAGED = _os.path.join(_os.path.dirname(_os.path.dirname(_os.path.dirname(_os.path.abspath(__file__)))), "baseline", "_ref")
-REFERENCE_ROOT = "/root/reference" if _os.path.isdir("/root/reference") else _STAGED
+# the checkout named by $PF_REFERENCE_ROOT, else the byte-for-byte copy oracle/pin/stage_reference.py staged in oracle/_ref
+_STAGED = _os.path.join(_os.path.dirname(_os.path.dirname(_os.path.dirname(_os.path.abspath(__file__)))), "oracle", "_ref")
+REFERENCE_ROOT = _os.environ.get("PF_REFERENCE_ROOT") or _STAGED
 
 
 def reference_available() -> bool:
@@ -213,7 +213,7 @@ class Attention(nn.Module):
 
 
 def install() -> None:
-    """Register the stubs and put /root/reference on sys.path."""
+    """Register the stubs and put REFERENCE_ROOT on sys.path."""
     import transformers  # noqa: F401  (must be imported before a version-less `accelerate` stub exists)
 
     d = _mod("diffusers")

@@ -93,8 +93,8 @@ def test_small_vae_matches_reference_golden(golden_dir):
     # tiled decode vs the reference's tiled golden
     vae.enable_tiling()
     out_t = vae.decode(z.to("cuda:0"), temporal_chunk=True, window_size=1, tile_sample_min_size=32).sample.float().cpu()
-    assert out_t.shape == g["tiled32"].shape
-    assert (out_t - g["tiled32"]).abs().max().item() < TOL_MAX_ABS
+    assert tuple(out_t.shape) == g["tiled32_shape"]
+    assert (out_t.flatten()[::g["tiled32_stride"]] - g["tiled32_sample"]).abs().max().item() < TOL_MAX_ABS
 
 
 def test_default_width_vae_matches_oracle():
