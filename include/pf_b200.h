@@ -320,6 +320,12 @@ PF_API int pf_softmax_rows(void* s_bf16, int64_t rows, int32_t cols, int64_t ld,
 PF_API int pf_pack_latent(const void* z, int32_t z_is_f32, int32_t b, int32_t c, int32_t t, int32_t h, int32_t w,
                           void* y_bf16, int32_t cpad, int32_t y_t_total, int32_t y_t_offset, const float* frame_scale,
                           const float* frame_shift, void* stream);
+/* uint8 video frames [B, T, H, W, C] (channels last) -> the encoder's conv_in input, channels-last bf16
+ * [B, y_t_total, H, W, cpad] at frame t + y_t_offset (behind the causal halo), channels >= C zero (cpad % 8 == 0).
+ * Each value is ((v / 255) - 0.5) / 0.5 in fp32, rounded once to bf16: ToTensor + Normalize(0.5, 0.5) in the reference's
+ * order (P:906-910, causal_video_vae_demo.ipynb), replacing the host-side float conversion and the device repack. */
+PF_API int pf_pack_frames_u8(const void* frames_u8, int32_t b, int32_t t, int32_t h, int32_t w, int32_t c, void* y_bf16,
+                             int32_t cpad, int32_t y_t_total, int32_t y_t_offset, void* stream);
 /* Cross-fade of neighbouring decoded tiles (blend_v / blend_h, V:397-407), tensors viewed as fp32 [outer, L, inner] with L the
  * blended axis: b[o, y, i] = a[o, la - extent + y, i] * (1 - y/extent) + b[o, y, i] * (y/extent) for y < extent (in place). */
 PF_API int pf_blend_tiles(const float* a, float* b, int64_t outer, int32_t la, int32_t lb, int64_t inner, int32_t extent,

@@ -20,8 +20,8 @@ SYMBOLS = [
     "pf_attn_build_group_masks", "pf_attn_fwd_masked",
     "pf_ln_modulate", "pf_small_linear", "pf_timestep_embedding",
     "pf_patchify", "pf_unpatchify", "pf_cfg_euler_step", "pf_stage_hop",
-    "pf_causal_conv3d", "pf_groupnorm_stats", "pf_groupnorm_apply", "pf_softmax_rows", "pf_pack_latent", "pf_blend_tiles",
-    "pf_ctx_create", "pf_ctx_destroy", "pf_ctx_record_begin", "pf_ctx_record_end", "pf_ctx_replay", "pf_dit_step_flux",
+    "pf_causal_conv3d", "pf_groupnorm_stats", "pf_groupnorm_apply", "pf_softmax_rows", "pf_pack_latent", "pf_pack_frames_u8",
+    "pf_blend_tiles", "pf_ctx_create", "pf_ctx_destroy", "pf_ctx_record_begin", "pf_ctx_record_end", "pf_ctx_replay", "pf_dit_step_flux",
     "pf_dit_step_mmdit", "pf_vae_decode_chunk",
     "pf_peer_alloc", "pf_peer_free", "pf_peer_export", "pf_peer_open", "pf_peer_close", "pf_peer_barrier", "pf_peer_bcast",
     "pf_debug_umma",
@@ -167,6 +167,8 @@ def load() -> C.CDLL:
     lib.pf_softmax_rows.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_int64, C.c_float, C.c_void_p]
     lib.pf_pack_latent.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                    C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.pf_pack_frames_u8.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p,
+                                      C.c_int32, C.c_int32, C.c_int32, C.c_void_p]
     _lib = lib
     return lib
 

@@ -166,6 +166,37 @@ __global__ void pack_latent_kernel(const T* __restrict__ z, int b, int c, int t,
   y[((((static_cast<size_t>(bb) * y_t_total + tt + y_t_offset) * h + hh) * w + ww)) * cpad + cc] = __float2bfloat16(v);
 }
 
+// uint8 frames [B, T, H, W, C] -> channels-last bf16 [B, y_t_total, H, W, cpad] at frame t + y_t_offset, in the order of
+// ToTensor + Normalize(0.5, 0.5) (P:906-910): ((v / 255) - 0.5) / 0.5 in fp32, channels >= C zero.  One thread per
+// 8-channel output vector (one 16-byte store).
+__global__ void __launch_bounds__(256)
+pack_frames_u8_kernel(const uint8_t* __restrict__ frames, int b, int t, int h, int w, int c, __nv_bfloat16* __restrict__ y,
+                      int cpad, int y_t_total, int y_t_offset) {
+  const long long idx = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  const int cvecs = cpad >> 3;
+  const long long total = static_cast<long long>(b) * t * h * w * cvecs;
+  if (idx >= total) return;
+  const int cv = static_cast<int>(idx % cvecs);
+  const long long pix = idx / cvecs;                    // ((bb * t + tt) * h + hh) * w + ww
+  const long long hw = static_cast<long long>(h) * w;
+  const long long frame = pix / hw;
+  const int bb = static_cast<int>(frame / t), tt = static_cast<int>(frame % t);
+  const uint8_t* src = frames + pix * c;
+  float o[8];
+#pragma unroll
+  for (int i = 0; i < 8; ++i) {
+    const int ch = cv * 8 + i;
+    o[i] = ch < c ? __fdiv_rn(__fsub_rn(__fdiv_rn(static_cast<float>(src[ch]), 255.f), 0.5f), 0.5f) : 0.f;
+  }
+  uint4 u;
+  u.x = pack_bf16x2(o[0], o[1]);
+  u.y = pack_bf16x2(o[2], o[3]);
+  u.z = pack_bf16x2(o[4], o[5]);
+  u.w = pack_bf16x2(o[6], o[7]);
+  const size_t yrow = (static_cast<size_t>(bb) * y_t_total + tt + y_t_offset) * hw + (pix - frame * hw);
+  reinterpret_cast<uint4*>(y + yrow * cpad)[cv] = u;
+}
+
 // Cross-fade of two neighbouring decoded tiles (blend_v / blend_h, V:397-407): tensors viewed as [outer, L, inner] with L the
 // blended axis; b[o, y, i] = a[o, La - extent + y, i] * (1 - y / extent) + b[o, y, i] * (y / extent) for y < extent.
 __global__ void blend_tiles_kernel(const float* __restrict__ a, float* __restrict__ b, long long outer, int la, int lb,
@@ -251,6 +282,18 @@ int pf_pack_latent(const void* z, int32_t z_is_f32, int32_t b, int32_t c, int32_
                                                                   static_cast<__nv_bfloat16*>(y), cpad, y_t_total,
                                                                   y_t_offset, frame_scale, frame_shift);
   return check_launch("pf_pack_latent");
+}
+
+int pf_pack_frames_u8(const void* frames, int32_t b, int32_t t, int32_t h, int32_t w, int32_t c, void* y, int32_t cpad,
+                      int32_t y_t_total, int32_t y_t_offset, void* stream) {
+  using namespace pf;
+  PF_REQUIRE(frames && y && b > 0 && t > 0 && h > 0 && w > 0 && c > 0 && cpad >= c && cpad % 8 == 0 && y_t_offset >= 0 &&
+                 y_t_offset + t <= y_t_total,
+             "pf_pack_frames_u8: bad arguments");
+  const long long total = static_cast<long long>(b) * t * h * w * (cpad / 8);
+  pack_frames_u8_kernel<<<static_cast<unsigned>((total + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+      static_cast<const uint8_t*>(frames), b, t, h, w, c, static_cast<__nv_bfloat16*>(y), cpad, y_t_total, y_t_offset);
+  return check_launch("pf_pack_frames_u8");
 }
 
 

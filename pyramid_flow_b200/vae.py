@@ -5,7 +5,9 @@ Call surface used by the pipeline (pyramid_dit_for_video_gen_pipeline.py:1221-12
     self.vae.decode(latents, temporal_chunk=True, window_size=w, tile_sample_min_size=s).sample    # [B, 3, T', H', W']
     self.vae.encode(image[:, :, None]).latent_dist.sample()                                        # i2v image latent
 
-plus `.device`, `.dtype`, `.to()`, `.enable_tiling()`.  Weights come from a state-dict in the reference key layout
+plus `.device`, `.dtype`, `.to()`, `.enable_tiling()`.  encode() also takes the reference's video arguments
+(`temporal_chunk`, `window_size`, `tile_sample_min_size`) with their meaning, and `encode_frames_u8` encodes uint8 video
+frames straight from a decoder.  Weights come from a state-dict in the reference key layout
 (`decoder.*`, `post_quant_conv.*`, and — when present — `encoder.*`, `quant_conv.*`; SURVEY.md §8b).  The encoder reuses the
 decoder's kernels; its down-samplers are the same implicit-GEMM conv with a strided TMA box (`stride_*` in pf_conv3d_desc).
 
@@ -17,8 +19,12 @@ at a time as the pipeline does):
   * mid-block attention -> 1x1x1 convs for q/k/out, `pf_gemm_bf16` for V^T, QK^T and PV, `pf_softmax_rows`
   * temporal chunking = the reference's feature cache (C:126-143): each 3x3x3 conv keeps the last two frames of its padded
     input and they become the halo of the next chunk; chunking is exact, so the chunk length is a memory knob only.
-Spatial tiling (V:468-519) is reproduced by decoding tiles independently and cross-fading them (`tile_sample_min_size`),
-but on 180 GB the un-tiled path is the default unless `enable_tiling()` was called, as in the reference.
+    The encoder's stride-2 temporal down-samplers read only the last cached frame in a later chunk (C:140-141), so an
+    encode is exact only when the window is a multiple of 2^(temporal down-samplers); other windows follow the reference's
+    rule and may return fewer latent frames.
+Spatial tiling (V:409-466, V:468-519) is reproduced by encoding / decoding tiles independently and cross-fading them
+(`tile_sample_min_size`), but on 180 GB the un-tiled path is the default unless `enable_tiling()` was called, as in the
+reference.
 """
 from __future__ import annotations
 
@@ -112,6 +118,7 @@ class B200CausalVAE(torch.nn.Module):
         self._cp = None                     # (group, rank, world) when context-parallel decode is on
         self._cp_ctx = None
         self.cp_frames_per_round = 4        # latent frames per rank per round (memory knob: ~6 GiB per frame at 768p)
+        self.encode_tile_overlap_factor = 0.25
         self.decode_tile_overlap_factor = 0.25
         dev = torch.device(device)
         self._dev = dev
@@ -240,7 +247,8 @@ class B200CausalVAE(torch.nn.Module):
 
     def _halo(self, cv: _Conv, buf: torch.Tensor, first: bool) -> None:
         """Fill the 2 leading frames of a 3x3x3 conv's input buffer from its cache (zeros for the first chunk) and
-        remember the last 2 frames of the padded input for the next chunk (reference C:126-143)."""
+        remember the last 2 frames of the padded input for the next chunk (reference C:126-143).  A stride-2 temporal conv
+        reads a later chunk's buffer from frame 1 (see _encode_chunk)."""
         if cv.kt == 1:
             return
         if self._cp is not None:
@@ -407,22 +415,31 @@ class B200CausalVAE(torch.nn.Module):
         self._conv(co, a, t, h, w, out=out, store_channels=cfg.out_channels, out_f32=2 if u8 else 1)
         return out
 
-    # ---- encoder (i2v image latent, P:911) ----------------------------------------------------------------------------
-    def _encode_sample(self, x: torch.Tensor) -> torch.Tensor:
-        """x: [1, C, T, H, W] (T = 1 + 8k, H and W multiples of 8) -> moments fp32 [T', h, w, 2*latent], whole clip as one
-        chunk (CausalVaeEncoder.forward D:149-198 with is_init_image=True, then quant_conv V:301)."""
+    # ---- encoder (i2v image latent P:911, video latents V:274-341) ---------------------------------------------------
+    def _encode_chunk(self, x: torch.Tensor, first: bool) -> torch.Tensor:
+        """One temporal chunk of one sample -> moments fp32 [T', h, w, 2*latent] (CausalVaeEncoder.forward D:149-198, then
+        quant_conv V:301).  x (on the device): [1, C, T, H, W] fp32 / bf16, or uint8 frames [T, H, W, C] normalised by
+        pf_pack_frames_u8.  `first` = the clip's first chunk: zero causal pad; later chunks continue from every 3x3x3 conv's
+        cache (C:126-143), so the whole clip as one chunk is the un-chunked encode."""
         cfg, dev = self.cfg, self.device
-        _, cx, t, h, w = x.shape
+        if x.dtype == torch.uint8:
+            t, h, w, cx = x.shape
+        else:
+            _, cx, t, h, w = x.shape
         n_blocks = len(cfg.enc_block_out_channels)
-        n_sp, n_tp = sum(cfg.enc_spatial_down_sample), sum(cfg.enc_temporal_down_sample)
+        n_sp = sum(cfg.enc_spatial_down_sample)
         assert h % (1 << n_sp) == 0 and w % (1 << n_sp) == 0, "height / width must be divisible by the spatial down-sampling"
-        assert (t - 1) % (1 << n_tp) == 0, "frames must be 1 + k * temporal down-sampling (V:315)"
         cin = self.convs["encoder.conv_in"]
         a = torch.empty(t + 2, h, w, cin.cin_p, device=dev, dtype=torch.bfloat16)
-        xx = x if x.dtype in (torch.float32, torch.bfloat16) else x.float()
-        _lib.check(_lib.load().pf_pack_latent(xx.contiguous().data_ptr(), int(xx.dtype == torch.float32), 1, cx, t, h, w,
-                                              a.data_ptr(), cin.cin_p, t + 2, 2, None, None, _lib.stream_ptr()), "pf_pack_latent")
-        self._halo(cin, a, True)
+        if x.dtype == torch.uint8:
+            _lib.check(_lib.load().pf_pack_frames_u8(x.contiguous().data_ptr(), 1, t, h, w, cx, a.data_ptr(), cin.cin_p, t + 2,
+                                                     2, _lib.stream_ptr()), "pf_pack_frames_u8")
+        else:
+            xx = x if x.dtype in (torch.float32, torch.bfloat16) else x.float()
+            _lib.check(_lib.load().pf_pack_latent(xx.contiguous().data_ptr(), int(xx.dtype == torch.float32), 1, cx, t, h, w,
+                                                  a.data_ptr(), cin.cin_p, t + 2, 2, None, None, _lib.stream_ptr()),
+                       "pf_pack_latent")
+        self._halo(cin, a, first)
         y = torch.empty(t, h, w, cin.cout_p, device=dev, dtype=torch.bfloat16)
         self._conv(cin, a, t, h, w, out=y)                                        # conv_in, D:152
         del a
@@ -431,12 +448,12 @@ class B200CausalVAE(torch.nn.Module):
             xb = None
             for j in range(cfg.enc_layers_per_block[i]):
                 last = j == cfg.enc_layers_per_block[i] - 1
-                y = self._resnet(f"encoder.down_blocks.{i}.resnets.{j}", y, True, halo_out=last and (sp or tp))
+                y = self._resnet(f"encoder.down_blocks.{i}.resnets.{j}", y, first, halo_out=last and (sp or tp))
                 if last and (sp or tp):
                     xb = y                                  # [t+2, h, w, c]: data in frames [2:]
             if sp:                                          # CausalDownsample2x: 3x3x3, stride (1,2,2), K:532-534
                 cv = self.convs[f"encoder.down_blocks.{i}.downsamplers.0.conv"]
-                self._halo(cv, xb, True)
+                self._halo(cv, xb, first)
                 off = 2 if tp else 0
                 h, w = h // 2, w // 2
                 y = torch.empty(t + off, h, w, cv.cout_p, device=dev, dtype=torch.bfloat16)
@@ -445,43 +462,131 @@ class B200CausalVAE(torch.nn.Module):
                 y = y[off:]
             if tp:                                          # CausalTemporalDownsample2x: 3x3x3, stride (2,1,1), K:536-538
                 cv = self.convs[f"encoder.down_blocks.{i}.temporal_downsamplers.0.conv"]
-                self._halo(cv, xb, True)
-                t_out = (t - 1) // 2 + 1                    # padded length t+2, kernel 3, stride 2
+                self._halo(cv, xb, first)
+                # a later chunk's input is [cache[-1:] ; chunk] (C:140-141): the older cached frame is skipped.  The cache
+                # _halo kept is still the last two frames of that input, whether or not the strided conv reads the last one.
+                src = xb if first else xb[1:]
+                assert src.shape[0] >= 3, "a later temporal chunk is too short for the stride-2 conv (window_size >= 2)"
+                t_out = (src.shape[0] - 3) // 2 + 1
                 y = torch.empty(t_out, h, w, cv.cout_p, device=dev, dtype=torch.bfloat16)
-                self._conv(cv, xb[: 2 * (t_out - 1) + 3], t_out, h, w, out=y)
+                self._conv(cv, src[: 2 * (t_out - 1) + 3], t_out, h, w, out=y)
                 t = t_out
-        y = self._resnet("encoder.mid_block.resnets.0", y, True)
+        y = self._resnet("encoder.mid_block.resnets.0", y, first)
         y = self._mid_attention(y, "encoder")
-        y = self._resnet("encoder.mid_block.resnets.1", y, True)
+        y = self._resnet("encoder.mid_block.resnets.1", y, first)
         co, qc = self.convs["encoder.conv_out"], self.convs["quant_conv"]
         a = torch.empty(t + 2, h, w, y.shape[-1], device=dev, dtype=torch.bfloat16)
         self._gn("encoder.conv_norm_out", y, a, 2, True)
-        self._halo(co, a, True)
+        self._halo(co, a, first)
         m = torch.zeros(t, h, w, qc.cin_p, device=dev, dtype=torch.bfloat16)      # padded channels must read as zero
         self._conv(co, a, t, h, w, out=m, store_channels=co.cout)                 # conv_out -> 2*latent channels
         out = torch.empty(t, h, w, qc.cout, device=dev, dtype=torch.float32)
         self._conv(qc, m, t, h, w, out=out, store_channels=qc.cout, out_f32=True)  # quant_conv (1x1x1), V:301
-        self._reset_caches()
         return out
+
+    @staticmethod
+    def chunk_bounds(n_frames: int, window_size: int):
+        """Temporal chunks [a, b) of chunk_encode / chunk_decode (V:311-327, V:347-360): the first window_size + 1 frames,
+        then full windows of window_size, then the remainder."""
+        init = min(n_frames, window_size + 1)
+        bounds, f = [(0, init)], init
+        while f < n_frames:
+            bounds.append((f, min(n_frames, f + window_size)))
+            f += window_size
+        return bounds
+
+    @staticmethod
+    def encode_tile_grid(height: int, width: int, tile_sample_min_size: int, overlap_factor: float = 0.25,
+                         downsample: int = 8):
+        """Tile geometry of tiled_encode (V:429-438): tile origins (rows, columns) in pixels, every tile_sample_min_size
+        wide (edge tiles are cut by the frame), the latent blend extent and the latent rows / columns kept per tile."""
+        tile_latent = int(tile_sample_min_size / downsample)
+        stride = int(tile_sample_min_size * (1 - overlap_factor))
+        extent = int(tile_latent * overlap_factor)
+        return list(range(0, height, stride)), list(range(0, width, stride)), extent, tile_latent - extent
+
+    @staticmethod
+    def _window(x: torch.Tensor, b: int, ts=slice(None), hs=slice(None), ws=slice(None)) -> torch.Tensor:
+        """Sample b, frames ts, rows hs, columns ws of a clip [B, C, T, H, W] (-> [1, C, t, h, w]) or of uint8 frames
+        [B, T, H, W, C] (-> [t, h, w, C])."""
+        return x[b, ts, hs, ws] if x.dtype == torch.uint8 else x[b:b + 1, :, ts, hs, ws]
+
+    def _encode_moments(self, x: torch.Tensor, window: int, hs=slice(None), ws=slice(None)) -> torch.Tensor:
+        """chunk_encode (V:311-341) of rows hs / columns ws of every sample, with `window` frames per chunk (the whole clip
+        when window >= T - 1): moments fp32 [B, T', h, w, 2*latent].  Chunks move to the device one at a time, so a clip on
+        the host never has to be resident on the device."""
+        n = x.shape[1] if x.dtype == torch.uint8 else x.shape[2]
+        n_tp = sum(self.cfg.enc_temporal_down_sample)
+        assert (n - 1) % (1 << n_tp) == 0, "frames must be 1 + k * temporal down-sampling (V:315)"
+        outs = []
+        for b in range(x.shape[0]):
+            self._reset_caches()
+            parts = [self._encode_chunk(self._window(x, b, slice(f0, f1), hs, ws).to(self.device), k == 0)
+                     for k, (f0, f1) in enumerate(self.chunk_bounds(n, window))]
+            self._reset_caches()
+            outs.append(torch.cat(parts, 0) if len(parts) > 1 else parts[0])
+        return torch.stack(outs, 0)
+
+    def _tiled_encode(self, x: torch.Tensor, window: int, tile_sample_min_size: int) -> torch.Tensor:
+        """tiled_encode (V:409-466): tiles encoded independently (chunked with `window`), fp32 moments cross-faded with the
+        tile above and to the left, then cropped -> [B, 2*latent, T', h, w]."""
+        hh, ww = (x.shape[2], x.shape[3]) if x.dtype == torch.uint8 else (x.shape[3], x.shape[4])
+        row0, col0, extent, limit = self.encode_tile_grid(hh, ww, tile_sample_min_size, self.encode_tile_overlap_factor,
+                                                          self.cfg.downsample_scale)
+        s = tile_sample_min_size
+        rows = [[self._encode_moments(x, window, slice(i, i + s), slice(j, j + s)).permute(0, 4, 1, 2, 3).contiguous()
+                 for j in col0] for i in row0]
+        result_rows = []
+        for i, row in enumerate(rows):
+            res = []
+            for j, tile in enumerate(row):
+                if i > 0:
+                    tile = _blend(rows[i - 1][j], tile, extent, 3)
+                if j > 0:
+                    tile = _blend(row[j - 1], tile, extent, 4)
+                res.append(tile[:, :, :, :limit, :limit])
+            result_rows.append(torch.cat(res, dim=4))
+        return torch.cat(result_rows, dim=3)
+
+    def _encode(self, x: torch.Tensor, temporal_chunk: bool, window_size: int, tile_sample_min_size: int):
+        """The control flow of CausalVideoVAE.encode (V:290-303): tiled when tiling is on and the frame is larger than the
+        tile, else chunked with temporal_chunk, else the whole clip as one chunk.  x: [B, C, T, H, W] or uint8 frames
+        [B, T, H, W, C], on the host or the device."""
+        _lib.require_device()
+        assert self.has_encoder, "this B200CausalVAE was built from a state-dict without encoder.* weights"
+        t, hh, ww = x.shape[1:4] if x.dtype == torch.uint8 else x.shape[2:5]
+        assert window_size >= 1 or not temporal_chunk, "window_size must be positive"
+        window = window_size if temporal_chunk else t
+        saved_cp, self._cp = self._cp, None
+        try:
+            if self.use_tiling and (ww > tile_sample_min_size or hh > tile_sample_min_size):
+                moments = self._tiled_encode(x, window, tile_sample_min_size)
+            else:
+                moments = self._encode_moments(x, window).permute(0, 4, 1, 2, 3)       # [B, T', h, w, 2C] -> [B, 2C, ...]
+        finally:
+            self._cp = saved_cp
+        return EncoderOutput(DiagonalGaussian(moments.to(self.dtype)))
 
     @torch.no_grad()
     def encode(self, x: torch.Tensor, return_dict: bool = True, is_init_image: bool = True, temporal_chunk: bool = False,
                window_size: int = 16, tile_sample_min_size: int = 256):
-        """CausalVideoVAE.encode (V:274-308), un-tiled and un-chunked (the pipeline encodes ONE image, P:911; chunking is
-        exact in the reference, so a clip is encoded whole): returns `.latent_dist` with mean / logvar / std / sample()."""
-        _lib.require_device()
-        assert self.has_encoder, "this B200CausalVAE was built from a state-dict without encoder.* weights"
-        assert is_init_image, "clips start with the image frame"
-        x = x.to(self.device)
-        saved_cp, self._cp = self._cp, None
-        try:
-            moments = torch.stack([self._encode_sample(x[i:i + 1]) for i in range(x.shape[0])], 0)   # [B, T', h, w, 2C]
-        finally:
-            self._cp = saved_cp
-        dist = DiagonalGaussian(moments.permute(0, 4, 1, 2, 3).to(self.dtype))
-        if not return_dict:
-            return (dist,)
-        return EncoderOutput(dist)
+        """CausalVideoVAE.encode (V:274-308): x [B, 3, T, H, W] (T = 1 + 8k) on the host or the device.  With
+        enable_tiling() and a frame larger than tile_sample_min_size the frame is encoded in tiles (tiled_encode,
+        V:409-466), otherwise in chunks of window_size frames with temporal_chunk (chunk_encode, V:311-341), otherwise whole.
+        is_init_image has no effect on the result, as in the reference.  Returns `.latent_dist` with mean / logvar / std /
+        sample()."""
+        out = self._encode(x, temporal_chunk, window_size, tile_sample_min_size)
+        return out if return_dict else (out.latent_dist,)
+
+    @torch.no_grad()
+    def encode_frames_u8(self, frames: torch.Tensor, temporal_chunk: bool = True, window_size: int = 16,
+                         tile_sample_min_size: int = 256) -> EncoderOutput:
+        """encode() of video frames as they are decoded from a file: uint8 [T, H, W, 3] or [B, T, H, W, 3], on the host or
+        the device.  ToTensor + Normalize(0.5, 0.5) (P:906-910) runs in pf_pack_frames_u8 on the device, and only uint8
+        tiles / chunks cross from the host.  Same tiling and chunking rules and result as encode() of the normalised
+        frames in bf16."""
+        assert frames.dtype == torch.uint8 and frames.dim() in (4, 5), "frames must be uint8 [(B,) T, H, W, C]"
+        return self._encode(frames if frames.dim() == 5 else frames[None], temporal_chunk, window_size, tile_sample_min_size)
 
     def _decode_sample_cp(self, z: torch.Tensor) -> torch.Tensor:
         """Context-parallel decode of one sample (schedule: cp_frame_split): per round every rank decodes its frame range as
@@ -529,13 +634,7 @@ class B200CausalVAE(torch.nn.Module):
             finally:
                 self._cp = saved
         self._reset_caches()
-        n = z.shape[2]
-        init = min(n, window_size + 1)
-        bounds = [(0, init)]
-        f = init
-        while f < n:
-            bounds.append((f, min(n, f + window_size)))
-            f += window_size
+        bounds = self.chunk_bounds(z.shape[2], window_size)
         if affine is None and not u8:
             outs = [self._decode_chunk(z[:, :, a:b], i == 0) for i, (a, b) in enumerate(bounds)]
         else:
